@@ -17,8 +17,8 @@ the same frame through the host-buffer call `sm_step_host_async` (H2D of every f
 records and refine logits inside the timed region, SAME flags as `value`); `roofline` = the tensor-core conv family
 (dominant kernel) timed per launch with CUDA events; `cpu_baseline` = the oracle port of the reference timed on all of
 this box's host cores; `parity_check` = max relative error of this run's outputs against the CPU oracle.
-The timed region is at least --min-seconds long (default 2 s): every reported step is repeated `passes_per_step`
-times inside it and all per-step figures are per pass.
+`value` times exactly --steps steps; the `e2e` region is at least --min-seconds long (default 2 s).
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/<name>.npy, see `dump_step_outputs`.
 """
 from __future__ import annotations
 
@@ -352,10 +352,13 @@ def run_gpu(args, rank, local_rank, world):
     m.template(z, slot0=0)
     m.template(z, slot0=B)
 
+    last = {}
+
     def step(i, mask_head=True):
         # the whole frame of siamese_track (tools/test.py:201-261) in one engine call, nothing leaves the device
-        return m.step(xs[i % 4], anchors_dev, window_dev, tsz_dev, PENALTY_K, WINDOW_INFLUENCE, refine=sharp,
-                      mask_head=sharp and mask_head)
+        last["out"] = m.step(xs[i % 4], anchors_dev, window_dev, tsz_dev, PENALTY_K, WINDOW_INFLUENCE, refine=sharp,
+                             mask_head=sharp and mask_head)
+        return last["out"]
 
     def barrier():
         torch.cuda.synchronize()
@@ -377,24 +380,19 @@ def run_gpu(args, rank, local_rank, world):
     warm = max(args.warmup, 3)
     for i in range(warm):
         step(i)
-    # size the timed region: at least --min-seconds, every reported step = `passes` passes over a batch
-    est_ms = timed(step, 3) / 3
-    passes = max(1, math.ceil(args.min_seconds * 1e3 / (est_ms * args.steps)))
-    if world > 1:
-        t = torch.tensor([passes], device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        passes = int(t.item())
-    n_pass = args.steps * passes
+    est_ms = timed(step, 3) / 3           # sizes the e2e region below
     l0 = m.launch_count
     t_start = time.perf_counter()
-    ms = timed(step, n_pass)
+    ms = timed(step, args.steps)
     t_end = time.perf_counter()
     launches = m.launch_count - l0
     clocks = sampler.stop(t_start, t_end) if sampler else None
-    fps = world * B * n_pass / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:   # before any later call overwrites the engine's output buffers
+        dump_step_outputs(args.dump_outputs, last["out"])
+    fps = world * B * args.steps / (ms * 1e-3)
     fps_skip = None
     if sharp:
-        n_skip = max(3, n_pass // 4)
+        n_skip = max(3, args.steps // 4)
         ms_skip = timed(lambda i: step(i, mask_head=False), n_skip)
         fps_skip = world * B * n_skip / (ms_skip * 1e-3)
 
@@ -546,15 +544,13 @@ def run_gpu(args, rank, local_rank, world):
     gfl = (GFLOP_SHARP if sharp else GFLOP_RPN).get(S, 0.0)
     result = {
         "metric": metric_name(args), "value": fps, "unit": "frames/s", "n_gpus": world, "steps": args.steps,
-        "warmup": warm, "ms_per_step": ms / n_pass, "higher_is_better": True, "scaling": "weak",
+        "warmup": warm, "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None,
         "dtype": "f16x3 (hi+lo split fp16 operands on tcgen05, f32 accumulate; f32 CUDA-core stem/xcorr/refine)"
                  if args.precision == "exact" else "f16 (single-pass tcgen05, f32 accumulate)",
         "data": "synthetic", "config": workload_config(args, B, world),
         "precision_mode": args.precision,
-        "passes_per_step": passes, "timed_region_s": ms * 1e-3,
-        "timing_note": f"the timed region covers steps x passes_per_step = {n_pass} passes over a batch "
-                       f"(>= {args.min_seconds} s); ms_per_step and value are per pass",
+        "timed_region_s": ms * 1e-3,
         "algorithmic_tflops": fps * gfl / 1e3,
         "value_skip_dead_mask_head": fps_skip,
         "e2e": {"value": e2e_fps, "unit": "frames/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
@@ -585,6 +581,26 @@ def run_gpu(args, rank, local_rank, world):
     print(json.dumps(result))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_ARRAY_BYTES = 8 << 20      # per array: Custom.step returns at most 7, so a dump stays under 64 MB
+
+
+def dump_step_outputs(path, out):
+    """Writes one step's outputs (the dict `Custom.step` returns) as path/<name>.npy: integer outputs as float64 (exact),
+    the rest as float32.  An array larger than DUMP_ARRAY_BYTES (the raw mask head: 635 MB at B=64) is written as
+    <name>_sample.npy, its elements at flat indices drawn from a generator seeded with 0: the same in every run."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for name, t in out.items():
+        if t is None:
+            continue
+        t = t.float() if t.is_floating_point() else t.double()
+        cap = DUMP_ARRAY_BYTES // t.element_size()
+        if t.numel() > cap:
+            idx = torch.randint(t.numel(), (cap,), generator=torch.Generator().manual_seed(0)).to(t.device)
+            name, t = name + "_sample", t.flatten()[idx]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
 
 
 def tracker_loop_rate(args, m, B, dev, seconds=1.5):
@@ -676,7 +692,7 @@ def main():
     ap.add_argument("--precision", default="exact", choices=["exact", "fast"])
     ap.add_argument("--rpn-only", action="store_true", default=None,
                     help="SiamRPN-only engine (experiments/siamrpn_resnet): step = track -> cls/loc")
-    ap.add_argument("--min-seconds", type=float, default=2.0, help="minimum length of every timed region")
+    ap.add_argument("--min-seconds", type=float, default=2.0, help="minimum length of the e2e timed region")
     ap.add_argument("--ref-batch", type=int, default=2, help="frames per step of each CPU reference worker")
     ap.add_argument("--cpu-threads", type=int, default=0, help="torch threads per CPU worker (0 = pick)")
     ap.add_argument("--cpu-seconds", type=float, default=10.0, help="length of the cpu_baseline sample")
@@ -686,11 +702,15 @@ def main():
     ap.add_argument("--no-verify", dest="verify", action="store_false", help="skip the oracle parity check")
     ap.add_argument("--traffic-file", default="r02_traffic.json")
     ap.add_argument("--dump-layers", default=None, help="write the per-launch CUDA-event table of one step here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (same arguments, same inputs)")
     # internal (cpu worker processes)
     ap.add_argument("--threads", type=int, default=8)
     ap.add_argument("--worker-id", type=int, default=0)
     ap.add_argument("--worker-seconds", type=float, default=0.0)
     args = ap.parse_args()
+    if args.steps < 1 and args.impl != "_cpu_worker":     # a CPU worker gets --steps 0 when it runs for --worker-seconds
+        ap.error("--steps must be at least 1")
     preset = PRESETS[args.config]
     if args.batch is None:
         args.batch = preset["batch"]

@@ -90,14 +90,27 @@ def sharp_383_golden(m):
                         corr=sub(m.corr_feature, 13), **feats, **ref)
 
 
+def sharp_seed11_golden(m):
+    """Sharp path at search 255 on the seed-11 inputs: cls, loc, 21 mask-head channels and the refine logits at the
+    border position (0, 24) — what tests/test_oracle.py::test_oracle_matches_reference_outputs compares against."""
+    from oracle.calibrate import synthetic_inputs
+    z, x = synthetic_inputs(11, 1)
+    m.template(z)
+    cls, loc, mask = m.track_mask(x)
+    np.savez_compressed(os.path.join(OUT, "sharp_b1_s255_seed11.npz"), cls=cls.numpy(), loc=loc.numpy(),
+                        mask_sub=mask[:, slice(0, 3969, 193)].numpy(), refine_0_24=m.track_refine((0, 24)).numpy())
+
+
 def main():
     from oracle.calibrate import calibrated_state_dict, synthetic_inputs
-    if "--only-383" in sys.argv:          # add the sharp@383 vectors without rewriting the other files
-        warnings.filterwarnings("ignore")
-        torch.set_num_threads(8)
-        with torch.no_grad():
-            sharp_383_golden(reference_model(calibrated_state_dict(0)))
-        return
+    only = {"--only-383": sharp_383_golden, "--only-seed11": sharp_seed11_golden}
+    for flag, fn in only.items():         # add one file's vectors without rewriting the other files
+        if flag in sys.argv:
+            warnings.filterwarnings("ignore")
+            torch.set_num_threads(8)
+            with torch.no_grad():
+                fn(reference_model(calibrated_state_dict(0)))
+            return
     warnings.filterwarnings("ignore")
     torch.set_num_threads(8)
     sd = calibrated_state_dict(0)
@@ -125,6 +138,7 @@ def main():
         cls3, loc3 = m.track(x3)
         np.savez_compressed(os.path.join(OUT, "rpn_b1_s383.npz"), cls=cls3.numpy(), loc=loc3.numpy())
         sharp_383_golden(m)
+        sharp_seed11_golden(m)
         # --- standalone depthwise xcorr (models/rpn.py:32-38)
         sys.path[:0] = [REF]
         from models.rpn import conv2d_dw_group

@@ -1,7 +1,6 @@
 """The oracle against (i) the golden vectors produced by the unmodified reference (oracle/make_golden.py),
-(ii) the live reference model when /root/reference is present, (iii) independent plain-loop restatements."""
+(ii) the reference's outputs on a second input at the tighter 1e-4, (iii) independent plain-loop restatements."""
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -12,7 +11,6 @@ from conftest import GOLDEN, assert_close
 from oracle.calibrate import synthetic_inputs
 from oracle.siammask_oracle import Oracle, nearest_upsample_index, xcorr_depthwise_loops
 
-REF = "/root/reference"
 # The golden vectors were produced on the build container's CPU.  The calibrated checkpoint is regenerated
 # from its seed wherever the tests run; a different CPU (other conv kernels in the calibration pass) moves
 # BN statistics by ~1e-7 and this seeded network amplifies perturbations ~100x, hence 1e-3 here.
@@ -108,18 +106,16 @@ def test_per_stream_refine_equals_per_sample_loop(calib_sd):
         assert_close(both[b:b + 1], o1.track_refine(pos), 1e-4, f"refine stream {b}")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present on this box")
-def test_oracle_matches_live_reference(calib_sd):
-    sys.path[:0] = [REF, os.path.join(REF, "experiments", "siammask_sharp")]
-    from custom import Custom
-    m = Custom(anchors={"stride": 8, "ratios": [0.33, 0.5, 1, 2, 3], "scales": [8], "round_dight": 0}).eval()
-    m.load_state_dict(calib_sd, strict=False)
+def test_oracle_matches_reference_outputs(calib_sd):
+    """The oracle against the unmodified reference model's own track_mask / track_refine outputs on the seed-11
+    inputs, recorded by `python -m oracle.make_golden --only-seed11` (21 of the 3969 mask-head channels)."""
+    g = _g("sharp_b1_s255_seed11.npz")
     z, x = synthetic_inputs(11, 1)
     o = Oracle(calib_sd)
     with torch.no_grad():
-        m.template(z); o.template(z)
-        ref = m.track_mask(x)
-        got = o.track_mask(x)
-        for a, b, n in zip(got, ref, ("cls", "loc", "mask")):
-            assert_close(a, b, 1e-4, n + " vs live reference")
-        assert_close(o.track_refine((0, 24)), m.track_refine((0, 24)), 1e-4, "refine vs live reference")
+        o.template(z)
+        cls, loc, mask = o.track_mask(x)
+        assert_close(cls, g["cls"], 1e-4, "cls vs reference")
+        assert_close(loc, g["loc"], 1e-4, "loc vs reference")
+        assert_close(mask[:, slice(0, 3969, 193)], g["mask_sub"], 1e-4, "mask vs reference")
+        assert_close(o.track_refine((0, 24)), g["refine_0_24"], 1e-4, "refine vs reference")
