@@ -70,7 +70,6 @@ struct GemmParams {
   int n_tiles, m_tiles;
   int staged;           // 1: epilogue goes smem -> TMA store (NHWC split outputs)
   int reverse_m;        // 1: walk the M tiles from the last to the first (see Engine::conv_into: L2 reuse)
-  int ncat;             // 1: exact mode issues A_hi x [B_hi; B_lo] as ONE MMA of N = 2*BLOCK_N (A_hi read from smem once)
   Epilogue ep;
 };
 
@@ -132,7 +131,6 @@ CUtensorMap make_map_tiled_nd(const __half* base, int rank, const uint64_t* dims
                               const uint32_t* box, int swizzle_bytes);
 
 // conv3x3_patch_sm100.cu : 3x3 / s1 / p1 / Cin == Cout in {64, 128} on a resident input patch (no im2col traffic)
-int patch_conv_mode();
 bool patch_conv_supported(const Act& in, const ConvGeom& g);
 void launch_conv3x3_patch(const Act& in, const ConvGeom& g, const __half* w_hi, const __half* w_lo, int w_ld,
                           const Epilogue& ep, int nsplit, int num_sms, cudaStream_t st);

@@ -23,8 +23,6 @@
 #include "common.cuh"
 #include "ptx.cuh"
 
-#include <cstdlib>
-
 namespace smk {
 
 namespace {
@@ -50,7 +48,6 @@ struct PatchParams {
   int tiles_per_img, num_tiles;
   int panel_bytes;         // one plane of one patch buffer incl. slack rows
   int patch_rows;          // (RO+2)*PW
-  int ncat;                // 1: hi*hi and hi*lo as ONE MMA of N = 2*CM over [B_hi; B_lo] (see conv_gemm_sm100.cu)
   Epilogue ep;
 };
 
@@ -180,7 +177,7 @@ __global__ void __launch_bounds__(P_THREADS, 1) conv3x3_patch_kernel(const __gri
       mbar_wait_guarded(&tempty[acc], acc_phase ^ 1);
       tcgen05_fence_after();
       const uint32_t tmem_d = tmem_base + acc * C::ACC_COLS;
-      uint32_t acc_main = 0, acc_lo = 0;
+      uint32_t acc_main = 0;
       for (int kb = 0; kb < NKB; ++kb, ++unit) {
         const int pbuf = unit & 1;
         const uint32_t pph = (unit >> 1) & 1;
@@ -195,33 +192,19 @@ __global__ void __launch_bounds__(P_THREADS, 1) conv3x3_patch_kernel(const __gri
           mbar_wait_guarded(&bfull[bstage], bphase);
           tcgen05_fence_after();
           const uint32_t b_hi = smem_u32(bring + bstage * C::B_STAGE_BYTES);
-          const uint64_t da_hi = umma_desc_kmajor<128>(a_hi0 + shift);
-          const uint64_t da_lo = umma_desc_kmajor<128>(a_lo0 + shift);
-          const uint64_t db_hi = umma_desc_kmajor<128>(b_hi);
-          const uint64_t db_lo = umma_desc_kmajor<128>(b_hi + C::B_TILE_BYTES);
+          const uint64_t da_hi = umma_desc_kmajor_sw128(a_hi0 + shift);
+          const uint64_t da_lo = umma_desc_kmajor_sw128(a_lo0 + shift);
+          const uint64_t db_hi = umma_desc_kmajor_sw128(b_hi);
           if (leader) {
-            if (NSPLIT == 2 && p.ncat != 0) {
-              // the lo weight tile follows the hi tile in the stage and the accumulators are adjacent TMEM columns:
-              // the shifted A_hi view crosses the smem port once for hi*hi and hi*lo together
+            // exact mode: the lo weight tile follows the hi tile in the stage and the accumulators are adjacent TMEM
+            // columns, so hi*hi and hi*lo are ONE MMA of N = 2*CM over [B_hi; B_lo] and the shifted A_hi view crosses
+            // the smem port once for both (see conv_gemm_sm100.cu)
 #pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                const uint64_t kadd = static_cast<uint64_t>(k * 2);
-                umma_f16(tmem_d, da_hi + kadd, db_hi + kadd, idesc_cat, acc_main);
-                acc_main = 1;
-                umma_f16(tmem_d + CM, da_lo + kadd, db_hi + kadd, idesc, 1u);
-              }
-            } else {
-#pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                const uint64_t kadd = static_cast<uint64_t>(k * 2);   // 32 bytes >> 4 in the start-address field
-                umma_f16(tmem_d, da_hi + kadd, db_hi + kadd, idesc, acc_main);
-                acc_main = 1;
-                if constexpr (NSPLIT == 2) {
-                  umma_f16(tmem_d + CM, da_hi + kadd, db_lo + kadd, idesc, acc_lo);   // order of the concatenated form
-                  acc_lo = 1;
-                  umma_f16(tmem_d + CM, da_lo + kadd, db_hi + kadd, idesc, 1u);
-                }
-              }
+            for (int k = 0; k < 4; ++k) {
+              const uint64_t kadd = static_cast<uint64_t>(k * 2);   // 32 bytes >> 4 in the start-address field
+              umma_f16(tmem_d, da_hi + kadd, db_hi + kadd, idesc_cat, acc_main);
+              acc_main = 1;
+              if constexpr (NSPLIT == 2) umma_f16(tmem_d + CM, da_lo + kadd, db_hi + kadd, idesc, 1u);
             }
             umma_commit(&bempty[bstage]);
             if (tap == 8) {
@@ -231,7 +214,6 @@ __global__ void __launch_bounds__(P_THREADS, 1) conv3x3_patch_kernel(const __gri
           }
           __syncwarp();
           acc_main = 1;
-          acc_lo = 1;
           if (++bstage == C::B_STAGES) { bstage = 0; bphase ^= 1; }
         }
       }
@@ -343,12 +325,6 @@ void launch_patch(const PatchParams& p, int num_sms, cudaStream_t st) {
 
 }  // namespace
 
-// SMB200_PATCH3X3: 0 = off (im2col kernel everywhere), 1 = on (default)
-int patch_conv_mode() {
-  static const int mode = [] { const char* e = getenv("SMB200_PATCH3X3"); return e ? atoi(e) : 1; }();
-  return mode;
-}
-
 bool patch_conv_supported(const Act& in, const ConvGeom& g) {
   if (!(g.KH == 3 && g.KW == 3 && g.stride == 1 && g.pad == 1 && g.dil == 1 && g.Cin == g.Cout)) return false;
   if (!(g.Cin == 64 || g.Cin == 128)) return false;
@@ -371,8 +347,6 @@ void launch_conv3x3_patch(const Act& in, const ConvGeom& g, const __half* w_hi, 
   p.patch_rows = (p.RO + 2) * p.PW;
   p.panel_bytes = (p.patch_rows + 2 * P_SLACK_ROWS) * 128;
   SMK_CHECK(p.panel_bytes % 1024 == 0, "patch panels must keep the 1024-byte swizzle alignment");
-  static const int no_ncat = [] { const char* e = getenv("SMB200_NO_NCAT"); return e ? atoi(e) : 0; }();
-  p.ncat = no_ncat == 0 ? 1 : 0;
   p.ep = ep;
   for (int s = 0; s < nsplit; ++s) {
     const __half* a = s == 0 ? in.hi : in.lo;

@@ -35,7 +35,7 @@
 #include "common.cuh"
 #include "ptx.cuh"
 
-#include <cstdlib>
+#include <algorithm>
 #include <cstring>
 #include <mutex>
 #include <unordered_map>
@@ -45,21 +45,20 @@ namespace smk {
 namespace {
 
 constexpr int BLOCK_M = 128;
-constexpr int CIN_GRAIN = 64;  // convs need Cin % 64 == 0 (both k-block widths divide it)
+constexpr int BLOCK_K = 64;     // k-block width in fp16 elements: one 128-byte swizzled row
+constexpr int CIN_GRAIN = 64;  // convs need Cin % 64 == 0 (whole k-blocks per filter tap)
 constexpr int UMMA_K = 16;
 constexpr int SMEM_LIMIT = 227 * 1024;
 constexpr int NUM_EPI_WARPS = 8;   // two per TMEM lane quarter, alternating 32-column chunks
 constexpr int NUM_THREADS = 64 + 32 * NUM_EPI_WARPS;
 
-// BK = k-block width in fp16 elements: 64 (128-byte swizzled rows) or 32 (64-byte rows, finer pipeline stages)
 // CG = CTAs per tile: 1, or 2 = a CTA pair (cluster of 2, tcgen05 cta_group::2) computing a 256 x BLOCK_N tile — each
 // CTA stages its own 128 A rows and HALF of the B rows, so smem fill and MMA operand reads per flop drop by a third.
-template <int BLOCK_N, int NSPLIT, int BK, int CG = 1>
+template <int BLOCK_N, int NSPLIT, int CG = 1>
 struct Cfg {
-  static constexpr int SWIZZLE = BK * 2;
-  static constexpr int A_TILE_BYTES = BLOCK_M * BK * 2;
+  static constexpr int A_TILE_BYTES = BLOCK_M * BLOCK_K * 2;
   static constexpr int B_ROWS = BLOCK_N / CG;           // B rows staged by one CTA
-  static constexpr int B_TILE_BYTES = B_ROWS * BK * 2;
+  static constexpr int B_TILE_BYTES = B_ROWS * BLOCK_K * 2;
   static constexpr int STAGE_BYTES = NSPLIT * (A_TILE_BYTES + B_TILE_BYTES);
   // epilogue staging: 8 warps x NSPLIT planes x (32 rows x 64 B)
   static constexpr int STG_TILE_BYTES = 32 * 64;
@@ -104,12 +103,11 @@ __device__ __forceinline__ int m_block(const GemmParams& p, int tile, int rank) 
   return (p.reverse_m ? groups - 1 - mb : mb) * CG + rank;
 }
 
-template <int BLOCK_N, int NSPLIT, int BK, int CG>
+template <int BLOCK_N, int NSPLIT, int CG>
 __global__ void __launch_bounds__(NUM_THREADS, 1) conv_gemm_kernel(const __grid_constant__ GemmParams p) {
-  using C = Cfg<BLOCK_N, NSPLIT, BK, CG>;
+  using C = Cfg<BLOCK_N, NSPLIT, CG>;
   constexpr int STAGES = C::STAGES;
   constexpr int CH = C::CH;
-  constexpr int BLOCK_K = BK;
   constexpr int A_TILE_BYTES = C::A_TILE_BYTES;
 
   extern __shared__ uint8_t smem_raw[];
@@ -251,8 +249,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_gemm_kernel(const __grid_
   } else if (warp == 1 && rank == 0) {
     // ===================== MMA issuer (pairs: the leader CTA issues for both) =====================
     constexpr uint32_t idesc = umma_idesc_f16(BLOCK_M * CG, BLOCK_N);
-    constexpr bool NCAT_OK = NSPLIT == 2 && CG == 1 && 2 * BLOCK_N <= 256;
-    constexpr uint32_t idesc_cat = umma_idesc_f16(BLOCK_M, NCAT_OK ? 2 * BLOCK_N : BLOCK_N);
+    // exact single-CTA tiles issue hi*hi and hi*lo as one MMA over [B_hi; B_lo] (see below); the pair tile keeps
+    // three MMAs per k-step, since its N = 256 leaves no room for the concatenated operand
+    constexpr bool NCAT = NSPLIT == 2 && CG == 1;
+    static_assert(!NCAT || 2 * BLOCK_N <= 256, "concatenated MMA: N <= 256");
+    constexpr uint32_t idesc_cat = umma_idesc_f16(BLOCK_M, NCAT ? 2 * BLOCK_N : BLOCK_N);
     auto wait_bar = [&](uint64_t* bar, uint32_t parity) {
       if constexpr (CG == 2) mbar_wait_guarded(bar, parity);
       else mbar_wait(bar, parity);
@@ -287,12 +288,12 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) conv_gemm_kernel(const __grid_
           const uint32_t a_hi = smem_u32(smem + stage * C::STAGE_BYTES);
           const uint32_t b_hi = a_hi + NSPLIT * A_TILE_BYTES;
           // descriptors once per k-block; the K steps add (16 elements * 2 B) >> 4 = 2 to the start-address field
-          const uint64_t da_hi0 = umma_desc_kmajor<C::SWIZZLE>(a_hi);
-          const uint64_t db_hi0 = umma_desc_kmajor<C::SWIZZLE>(b_hi);
-          const uint64_t da_lo0 = umma_desc_kmajor<C::SWIZZLE>(a_hi + A_TILE_BYTES);
-          const uint64_t db_lo0 = umma_desc_kmajor<C::SWIZZLE>(b_hi + C::B_TILE_BYTES);
+          const uint64_t da_hi0 = umma_desc_kmajor_sw128(a_hi);
+          const uint64_t db_hi0 = umma_desc_kmajor_sw128(b_hi);
+          const uint64_t da_lo0 = umma_desc_kmajor_sw128(a_hi + A_TILE_BYTES);
+          const uint64_t db_lo0 = umma_desc_kmajor_sw128(b_hi + C::B_TILE_BYTES);
           if (leader) {
-            if (NCAT_OK && p.ncat != 0 && !ident) {
+            if (NCAT && !ident) {
               // The B_lo tile follows the B_hi tile in the stage, so [B_hi; B_lo] is one K-major operand of 2*BLOCK_N
               // rows and the two accumulators are adjacent TMEM columns: A_hi x [B_hi; B_lo] is ONE MMA (hi*hi ->
               // acc0, hi*lo -> acc1) and A_hi crosses the shared-memory port once instead of twice (operand reads
@@ -614,8 +615,6 @@ template <typename F>
 CUtensorMap cached_map(const MapKey& key, F&& encode) {
   static std::mutex mu;
   static std::unordered_map<MapKey, CUtensorMap, MapKeyHash> cache;
-  static const bool off = getenv("SMB200_NO_MAP_CACHE") != nullptr;
-  if (off) return encode();
   int dev = 0;
   cudaGetDevice(&dev);
   MapKey k = key;
@@ -635,10 +634,9 @@ CUtensorMap make_map_2d_raw(const __half* base, uint64_t inner, uint64_t outer, 
   cuuint64_t strides[1] = {inner * sizeof(__half)};
   cuuint32_t box[2] = {box_inner, box_outer};
   cuuint32_t estr[2] = {1, 1};
-  // operand tiles: the swizzle span equals the k-block row (64 fp16 -> 128 B, 32 fp16 -> 64 B)
-  const CUtensorMapSwizzle sw = box_inner == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
+  // operand tiles: the swizzle span equals the k-block row (64 fp16 = 128 B)
   CUresult r = driver_api().tiled(&m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<__half*>(base), dims, strides,
-                                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
+                                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   SMK_CHECK(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed, code " + std::to_string((int)r));
   return m;
@@ -669,7 +667,7 @@ CUtensorMap make_map_epilogue(const __half* base, uint64_t cout, uint64_t m) {
   return cached_map(k, [&] { return make_map_epilogue_raw(base, cout, m); });
 }
 
-CUtensorMap make_map_im2col_raw(const __half* base, const Act& in, const ConvGeom& g, int bk) {
+CUtensorMap make_map_im2col_raw(const __half* base, const Act& in, const ConvGeom& g) {
   CUtensorMap m;
   cuuint64_t dims[4] = {(cuuint64_t)in.C, (cuuint64_t)in.W, (cuuint64_t)in.H, (cuuint64_t)in.B};
   cuuint64_t strides[3] = {(cuuint64_t)in.C * 2, (cuuint64_t)in.W * in.C * 2, (cuuint64_t)in.H * in.W * in.C * 2};
@@ -680,8 +678,7 @@ CUtensorMap make_map_im2col_raw(const __half* base, const Act& in, const ConvGeo
   cuuint32_t estr[4] = {1, (cuuint32_t)g.stride, (cuuint32_t)g.stride, 1};
   const DriverApi& api = driver_api();
   CUresult r = api.im2col(&m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<__half*>(base), dims, strides, lower,
-                          upper, bk, BLOCK_M, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          bk == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
+                          upper, BLOCK_K, BLOCK_M, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   SMK_CHECK(r == CUDA_SUCCESS, "cuTensorMapEncodeIm2col failed, code " + std::to_string((int)r));
   // Same small-tensor descriptor fix-up CuTe applies for drivers <= 13.1
@@ -691,19 +688,19 @@ CUtensorMap make_map_im2col_raw(const __half* base, const Act& in, const ConvGeo
   return m;
 }
 
-CUtensorMap make_map_im2col(const __half* base, const Act& in, const ConvGeom& g, int bk) {
+CUtensorMap make_map_im2col(const __half* base, const Act& in, const ConvGeom& g) {
   MapKey k{};
   k.v[0] = 3; k.v[1] = (uint64_t)base;
   k.v[2] = ((uint64_t)in.B << 32) | (uint32_t)in.H; k.v[3] = ((uint64_t)in.W << 32) | (uint32_t)in.C;
   k.v[4] = ((uint64_t)g.KH << 32) | (uint32_t)g.KW; k.v[5] = ((uint64_t)g.stride << 32) | (uint32_t)g.pad;
-  k.v[6] = ((uint64_t)g.dil << 32) | (uint32_t)bk;
-  return cached_map(k, [&] { return make_map_im2col_raw(base, in, g, bk); });
+  k.v[6] = (uint64_t)g.dil;
+  return cached_map(k, [&] { return make_map_im2col_raw(base, in, g); });
 }
 
-template <int BLOCK_N, int NSPLIT, int BK = 64, int CG = 1>
+template <int BLOCK_N, int NSPLIT, int CG = 1>
 void launch_cfg(const GemmParams& p, int num_sms, cudaStream_t st) {
-  using C = Cfg<BLOCK_N, NSPLIT, BK, CG>;
-  auto kern = conv_gemm_kernel<BLOCK_N, NSPLIT, BK, CG>;
+  using C = Cfg<BLOCK_N, NSPLIT, CG>;
+  auto kern = conv_gemm_kernel<BLOCK_N, NSPLIT, CG>;
   static unsigned long long attr_done = 0;
   ensure_dynamic_smem(kern, C::SMEM_BYTES, attr_done);
   const int tiles = ((p.m_tiles + CG - 1) / CG) * p.n_tiles;
@@ -817,48 +814,34 @@ void launch_gemm_multi(const GemmInput* convs, int nconv, const Act* residual, i
   p.Cout = g0.Cout;
   p.Ho = Ho;
   p.Wo = Wo;
-  // Tile choice.  fast: 128 x 256.  exact: 128 x 128 with two double-buffered TMEM accumulator pairs, or — when the
-  // main loop is long enough to amortise a non-overlapped epilogue (>= 24 k-blocks) — 128 x 256 with a single
-  // accumulator stage and two 96 KB ring stages.  The SM's shared-memory port (128 B/clk) carries both the TMA fills
-  // and the operand reads of every tcgen05.mma; per k-block a 128 x 128 exact tile moves 64 KB in + 96 KB out of smem
-  // for 768 MMA-clocks (208 B/clk -> <= 61 % tensor duty, 63-66 % measured), the 128 x 256 tile 96 + 144 KB for 1536
-  // (156 B/clk -> <= 82 %).  Measured on B200 (profiles/r01_tile_ab.md): layer3.0 conv3+downsample 1.45 -> 1.16 ms,
-  // 3x3 convs -10..-17 %, short-K 1x1 layers +8..+35 % slower (they stay on 128 x 128).  32-wide k-blocks (64 B
-  // rows) were slower everywhere.  SMB200_EXACT_N256: 0 = never wide, 1 = default rule, 3 = always wide.
-  static const int n256 = [] { const char* e = getenv("SMB200_EXACT_N256"); return e ? atoi(e) : 1; }();
-  static const int wide_kb = [] { const char* e = getenv("SMB200_WIDE_KB"); return e ? atoi(e) : 24; }();
+  // Tile choice.  fast: 128 x min(Cout, 256), single CTA.  exact: 128 x min(Cout, 128) with two double-buffered TMEM
+  // accumulator pairs, or — when the main loop is long enough to amortise a non-overlapped epilogue (>= kPairMinKb
+  // k-blocks) — a 256 x 256 CTA-pair tile with a single accumulator stage.  The SM's shared-memory port (128 B/clk)
+  // carries both the TMA fills and the operand reads of every tcgen05.mma; per k-block a 128 x 128 exact tile moves
+  // 64 KB in + 96 KB out of smem for 768 MMA-clocks (208 B/clk -> <= 61 % tensor duty, 63-66 % measured), a 128 x 256
+  // tile 96 + 144 KB for 1536 (156 B/clk -> <= 82 %).  Measured on B200 (profiles/r01_tile_ab.md): layer3.0
+  // conv3+downsample 1.45 -> 1.16 ms, 3x3 convs -10..-17 %, short-K 1x1 layers +8..+35 % slower (they stay on
+  // 128 x 128).  32-wide k-blocks (64 B rows) were slower everywhere.
+  // A CTA pair (cluster of 2, tcgen05 cta_group::2) stages its own 128 A rows per CTA and half of the B rows, so fills
+  // and operand reads through the smem port drop by a third (104 B/clk for the exact 256-wide tile).  Measured
+  // (profiles/r01_tile_ab.md): exact long-K layers -4..-9 %; fast 256-wide pairs +5..+12 % slower (not smem-bound);
+  // 256 x 128 pairs on the short-K exact layers neutral to slower (lock-step epilogues).
+  // The wide tile is taken only when the 128 x 128 tiling fills the machine anyway (small batches — B=1: 64 tiles —
+  // are latency bound and want as many CTAs as they can get), and only for NHWC split outputs: the 3969-channel NCHW
+  // mask head (K = 256) is slower on wide or pair tiles, its scalar-store epilogue needs the overlap (DESIGN.md §8).
+  constexpr int kPairMinKb = 24;
   int total_kb = residual != nullptr ? 2 : 0;
-  for (int i = 0; i < nconv; ++i) total_kb += convs[i].g.KH * convs[i].g.KW * convs[i].g.Cin / 64;
-  // ... and only when the 128 x 128 tiling would fill the machine anyway: small batches (B=1: 64 tiles) are latency
-  // bound and want as many CTAs as they can get
+  for (int i = 0; i < nconv; ++i) total_kb += convs[i].g.KH * convs[i].g.KW * convs[i].g.Cin / BLOCK_K;
   const long long narrow_tiles = (long long)((p.M + BLOCK_M - 1) / BLOCK_M) * (cout_pad / 128);
-  // NCHW fp32 outputs (the 3969-channel mask head: K = 256, 128 x 128 tiles re-stream 64 KB of operands per k-block
-  // and sit at the L2 -> SM fabric limit): SMB200_NCHW_WIDE=1 lets them take the 256-wide (pair) tile as well
-  static const int nchw_wide = [] { const char* e = getenv("SMB200_NCHW_WIDE"); return e ? atoi(e) : 0; }();
-  const bool wide_nchw = nchw_wide != 0 && nsplit == 2 && cout_pad >= 1024 && ep.out_mode == OUT_NCHW_F32 &&
-                         narrow_tiles >= num_sms;
-  const bool wide_exact = (nsplit == 2 && cout_pad >= 256 && ep.out_mode == OUT_NHWC_SPLIT &&
-                           (n256 == 3 || (n256 == 1 && total_kb >= wide_kb && narrow_tiles >= num_sms))) || wide_nchw;
-  const int block_n = cout_pad < 256 ? cout_pad : (nsplit == 2 && !wide_exact ? 128 : 256);
-  const int bk = 64;
-  // CTA pairs (cluster of 2, tcgen05 cta_group::2, 256 x 256 tiles): each CTA stages its own 128 A rows and half of
-  // the B rows, so fills and operand reads through the smem port drop by a third (104 B/clk for the exact tile).
-  // Measured (profiles/r01_tile_ab.md): exact long-K layers -4..-9 %; fast mode +5..+12 % slower (not smem-bound:
-  // stays single-CTA); 256 x 128 pairs on the short-K exact layers are neutral to slower (lock-step epilogues).
-  // SMB200_CTA_PAIR: 0 = never, 1 = default rule (exact 256-wide tiles), 2 = also the exact 128-wide tiles,
-  // 3 = also the fast 256-wide tiles.
-  static const int pair_mode = [] { const char* e = getenv("SMB200_CTA_PAIR"); return e ? atoi(e) : 1; }();
-  const int cg = (pair_mode >= 1 && wide_exact) || (pair_mode >= 2 && block_n == 128 && nsplit == 2) ||
-                         (pair_mode >= 3 && block_n == 256)
-                     ? 2 : 1;
+  const bool pair = nsplit == 2 && cout_pad >= 256 && ep.out_mode == OUT_NHWC_SPLIT && total_kb >= kPairMinKb &&
+                    narrow_tiles >= num_sms;
+  const int block_n = pair ? 256 : std::min(cout_pad, nsplit == 2 ? 128 : 256);
+  const int cg = pair ? 2 : 1;
   SMK_CHECK(cout_pad % block_n == 0, "cout_pad must be a multiple of the N tile");
   if (ep.out_mode != OUT_NCHW_F32) SMK_CHECK(g0.Cout == cout_pad, "NHWC outputs need Cout to match the padded tile width");
   p.n_tiles = cout_pad / block_n;
   p.m_tiles = (p.M + BLOCK_M - 1) / BLOCK_M;
   p.reverse_m = reverse_m ? 1 : 0;
-  // SMB200_NO_NCAT=1: issue hi*hi and hi*lo as two MMAs again (A/B runs)
-  static const int no_ncat = [] { const char* e = getenv("SMB200_NO_NCAT"); return e ? atoi(e) : 0; }();
-  p.ncat = (nsplit == 2 && cg == 1 && 2 * block_n <= 256 && no_ncat == 0) ? 1 : 0;
   p.nseg = 0;
   for (int i = 0; i < nconv; ++i) {
     const ConvGeom& g = convs[i].g;
@@ -869,7 +852,7 @@ void launch_gemm_multi(const GemmInput* convs, int nconv, const Act* residual, i
     SMK_CHECK(nsplit == 1 || (in.lo != nullptr && w_lo != nullptr), "exact mode needs lo planes");
     GemmSegment& sg = p.seg[p.nseg++];
     sg.kind = 0;
-    sg.cblks = g.Cin / bk;
+    sg.cblks = g.Cin / BLOCK_K;
     sg.num_kb = g.KH * g.KW * sg.cblks;
     sg.KW = g.KW;
     sg.stride = g.stride;
@@ -880,7 +863,7 @@ void launch_gemm_multi(const GemmInput* convs, int nconv, const Act* residual, i
     SMK_CHECK(sg.b_col0 % 64 == 0 && sg.b_col0 + g.KH * g.KW * g.Cin <= w_ld, "weight column range");
     for (int s = 0; s < nsplit; ++s) {
       const __half* a = s == 0 ? in.hi : in.lo;
-      sg.tmA[s] = sg.mode == 0 ? make_map_2d(a, g.Cin, (uint64_t)in.M(), bk, BLOCK_M) : make_map_im2col(a, in, g, bk);
+      sg.tmA[s] = sg.mode == 0 ? make_map_2d(a, g.Cin, (uint64_t)in.M(), BLOCK_K, BLOCK_M) : make_map_im2col(a, in, g);
     }
     if (nsplit == 1) sg.tmA[1] = sg.tmA[0];
   }
@@ -893,18 +876,18 @@ void launch_gemm_multi(const GemmInput* convs, int nconv, const Act* residual, i
     GemmSegment& sg = p.seg[p.nseg++];
     sg.kind = 1;
     sg.mode = 0;
-    sg.num_kb = block_n / bk;
+    sg.num_kb = block_n / BLOCK_K;
     sg.cblks = sg.KW = sg.stride = sg.dil = 1;
     sg.pad = 0;
     sg.b_col0 = res_col0;
     for (int s = 0; s < nsplit; ++s)
-      sg.tmA[s] = make_map_2d(s == 0 ? residual->hi : residual->lo, g0.Cout, (uint64_t)p.M, bk, BLOCK_M);
+      sg.tmA[s] = make_map_2d(s == 0 ? residual->hi : residual->lo, g0.Cout, (uint64_t)p.M, BLOCK_K, BLOCK_M);
     if (nsplit == 1) sg.tmA[1] = sg.tmA[0];
     ep.res_hi = ep.res_lo = nullptr;       // accumulated by the MMA, not by the epilogue
   }
   if (p.nseg == 1) p.seg[1] = p.seg[0];
   for (int s = 0; s < nsplit; ++s)
-    p.tmB[s] = make_map_2d(s == 0 ? w_hi : w_lo, (uint64_t)w_ld, cout_pad, bk, block_n / cg);
+    p.tmB[s] = make_map_2d(s == 0 ? w_hi : w_lo, (uint64_t)w_ld, cout_pad, BLOCK_K, block_n / cg);
   if (nsplit == 1) p.tmB[1] = p.tmB[0];
   // NHWC split outputs go through smem + TMA stores; an epilogue-side residual (no diagonal block) needs the
   // direct path
@@ -927,16 +910,10 @@ void launch_gemm_multi(const GemmInput* convs, int nconv, const Act* residual, i
     SMK_DISPATCH(16)
     SMK_DISPATCH(32)
     SMK_DISPATCH(64)
-    case 128:
-      if (nsplit == 2 && cg == 2) launch_cfg<128, 2, 64, 2>(p, num_sms, st);
-      else if (nsplit == 2) launch_cfg<128, 2>(p, num_sms, st);
-      else launch_cfg<128, 1>(p, num_sms, st);
-      break;
-    case 256:
-      if (nsplit == 1 && cg == 2) launch_cfg<256, 1, 64, 2>(p, num_sms, st);
-      else if (nsplit == 1) launch_cfg<256, 1>(p, num_sms, st);
-      else if (cg == 2) launch_cfg<256, 2, 64, 2>(p, num_sms, st);
-      else launch_cfg<256, 2, 64>(p, num_sms, st);
+    SMK_DISPATCH(128)
+    case 256:   // exact mode reaches the 256-wide tile only as a CTA pair
+      if (nsplit == 2) launch_cfg<256, 2, 2>(p, num_sms, st);
+      else launch_cfg<256, 1>(p, num_sms, st);
       break;
     default: SMK_CHECK(false, "unsupported N tile");
   }

@@ -86,7 +86,7 @@ struct Arena {
 };
 
 // One execution lane: its own workspace, stream set and cached per-step tensors.  A batch of >= 2 * kLaneMinB streams
-// is split over two (SMB200_LANES: up to kMaxLanes) lanes that run concurrently (streams are independent): the persistent GEMM kernels of one lane
+// is split over two lanes that run concurrently (streams are independent): the persistent GEMM kernels of one lane
 // fill the SMs the other lane's kernels leave idle in their last wave and in the low-occupancy refine tail.
 struct Lane {
   Arena search, refine;
@@ -95,7 +95,7 @@ struct Lane {
   cudaStream_t aux[3] = {nullptr, nullptr, nullptr};
   int cap_B = 0;                               // largest batch this lane's arenas were sized for
 };
-constexpr int kMaxLanes = 4;
+constexpr int kMaxLanes = 2;                   // 3 or 4 lanes measured slower than 2 (DESIGN.md §5)
 constexpr int kLaneMinB = 8;                   // a lane gets at least this many streams (below 2 x 8: one lane)
 
 }  // namespace
@@ -216,9 +216,9 @@ class Engine {
   Arena templ_arena_;
   Lane lanes_[kMaxLanes];
   Lane* cur_ = &lanes_[0];             // lane whose schedule is being enqueued
-  int n_lanes_ = 1;                    // SMB200_LANES (default 2), capped by max_batch / kLaneMinB
+  int n_lanes_ = 1;                    // kMaxLanes, capped by max_batch / kLaneMinB
   int split_n_ = 1;                    // how the last track divided its batch: lane l got streams
-  int split_off_[kMaxLanes + 1] = {0, 0, 0, 0, 0};   //   [split_off_[l], split_off_[l + 1])
+  int split_off_[kMaxLanes + 1] = {0, 0, 0};   //   [split_off_[l], split_off_[l + 1])
   // per-slot template caches: [branch][slot][5][5][256] split planes, and zf for export
   __half* kcache_hi_ = nullptr;
   __half* kcache_lo_ = nullptr;
@@ -271,7 +271,7 @@ class Engine {
     cudaGraphExec_t exec = nullptr;
     std::map<std::string, Act> named[kMaxLanes];
     int split_n = 1;
-    int split_off[kMaxLanes + 1] = {0, 0, 0, 0, 0};
+    int split_off[kMaxLanes + 1] = {0, 0, 0};
     int last_B = 0;
     bool have_mask_feats = false;
     int64_t launches = 0;
@@ -567,11 +567,7 @@ void Engine::construct(const sm_config& cfg) {
   }
 
   // workspace sizes: dry-run the schedule with a measuring arena
-  {
-    const char* e = std::getenv("SMB200_LANES");
-    const int want = e != nullptr ? std::max(1, std::min(kMaxLanes, atoi(e))) : 2;
-    n_lanes_ = lanes_for(want, cfg.max_batch);
-  }
+  n_lanes_ = lanes_for(kMaxLanes, cfg.max_batch);
   // the largest chunk each lane can be handed over all batch sizes this engine accepts (lane 0: the whole batch,
   // when profiling)
   lanes_[0].cap_B = cfg.max_batch;
@@ -1096,11 +1092,10 @@ void Engine::conv_into(const Act& in, const ConvW& Lw, Epilogue ep, cudaStream_t
     const Act* big = &in;
     if (in2 != nullptr && in2->numel() > big->numel()) big = in2;
     if (res != nullptr && res->numel() > big->numel()) big = res;
-    static const bool no_reverse = std::getenv("SMB200_NO_REVERSE") != nullptr;   // A/B switch for measurements
     // bottleneck conv2 (3x3 / s1 / p1, 64 or 128 channels): resident-patch kernel, walks its tiles front to back
-    const bool use_patch = patch_conv_mode() != 0 && in2 == nullptr && res == nullptr &&
+    const bool use_patch = in2 == nullptr && res == nullptr &&
                            ep.out_mode == OUT_NHWC_SPLIT && patch_conv_supported(in, Lw.g);
-    const bool reverse = !use_patch && !no_reverse && end_of(*big) > 0;
+    const bool reverse = !use_patch && end_of(*big) > 0;
     const int now_end = reverse ? -1 : +1;
     last_end_[in.hi] = now_end;
     if (in2 != nullptr) last_end_[in2->hi] = now_end;
@@ -1303,8 +1298,7 @@ void Engine::track_lane(int slot0, int B, const float* x, float* cls, float* loc
   const int nb = (want_feats || want_mask_head) ? 3 : 2;
   float* outs[3] = {cls, loc, mask};
   // all branches wanted: their conv_search layers run as ONE GEMM over xf (N = 256 x branches)
-  static const bool no_cat = std::getenv("SMB200_NO_SEARCH_CAT") != nullptr;
-  const bool use_cat = nb == n_branches_ && cfg_.backend == SM_BACKEND_TENSOR && !no_cat;
+  const bool use_cat = nb == n_branches_ && cfg_.backend == SM_BACKEND_TENSOR;
   Act cs_all;
   if (use_cat) cs_all = conv(xf, L(kSearchCat), true, nullptr, search_arena, st);
   for (int br = 0; br < nb; ++br) {
@@ -1769,7 +1763,7 @@ static void conv2d_op(const float* x, const float* w, const float* scale, const 
   SMK_CUDA(cudaGetDevice(&dev));
   SMK_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   (void)Ho; (void)Wo;
-  if (use_gemm && patch_conv_mode() != 0 && patch_conv_supported(in, g)) {
+  if (use_gemm && patch_conv_supported(in, g)) {
     // the engine runs this geometry on the resident-patch kernel (NHWC split output): same here, then export
     Act o;
     o.B = B; o.H = Ho; o.W = Wo; o.C = Cout;

@@ -246,19 +246,6 @@ __device__ __forceinline__ uint64_t umma_desc_kmajor_sw128(uint32_t smem_addr) {
   d |= static_cast<uint64_t>(2) << 61;            // SWIZZLE_128B
   return d;
 }
-// Same for a swizzle span of SW bytes per row (128: 64 fp16 per row, layout code 2; 64: 32 fp16, code 4):
-// 8-row groups are 8*SW bytes apart.
-template <int SW>
-__device__ __forceinline__ uint64_t umma_desc_kmajor(uint32_t smem_addr) {
-  static_assert(SW == 128 || SW == 64, "swizzle span");
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr & 0x3FFFF) >> 4);
-  d |= static_cast<uint64_t>(1) << 16;
-  d |= static_cast<uint64_t>((8 * SW) >> 4) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(SW == 128 ? 2 : 4) << 61;
-  return d;
-}
 // Instruction descriptor, kind::f16: fp16 A/B (K-major both), fp32 D, M x N tile.
 __host__ __device__ constexpr uint32_t umma_idesc_f16(int M, int N) {
   return (1u << 4)                                   // c_format = F32

@@ -1111,8 +1111,7 @@ void launch_xcorr_nchw_f32(const float* x, const float* k, float* out, int plane
                            cudaStream_t st) {
   SMK_CHECK(H >= kh && W >= kw && planes > 0, "xcorr shapes");
   // bulk-copy pipeline (xcorr_bulk_sm100.cu) for whole tiles of planes; the one-warp-per-plane kernel takes the rest
-  static const bool no_bulk = getenv("SMB200_XCORR_NO_BULK") != nullptr;
-  const int done = no_bulk ? 0 : launch_xcorr_bulk_f32(x, k, out, planes, H, W, kh, kw, st);
+  const int done = launch_xcorr_bulk_f32(x, k, out, planes, H, W, kh, kw, st);
   if (done >= planes) return;
   x += (size_t)done * H * W;
   k += (size_t)done * kh * kw;

@@ -75,45 +75,6 @@ def test_conv_simt_reference(case):
     assert_close(out, ref, 2e-5, "simt " + case[0])
 
 
-_VARIANT_SCRIPT = """
-import sys
-sys.path[:0] = [{tests!r}, {root!r}]
-import test_gpu_ops as t
-from conftest import assert_close
-import siammask_b200 as smb
-for c in t.CONV_CASES:
-    if c[0] not in {names!r}:
-        continue
-    for prec, tol, seed in (("exact", 2e-5, 0), ("fast", 3e-3, 1)):
-        x, w, scale, shift, ref, (s, p, d) = t._case(c, seed=seed)
-        out = smb.conv2d(x.cuda(), w, scale, shift, s, p, d, relu=True, backend="tensor", precision=prec)
-        assert_close(out, ref.relu(), tol, prec + " " + c[0])
-print("variants ok")
-"""
-
-
-@pytest.mark.parametrize("env", [{"SMB200_CTA_PAIR": "0"}, {"SMB200_CTA_PAIR": "3"},
-                                 {"SMB200_CTA_PAIR": "2", "SMB200_EXACT_N256": "0"},
-                                 {"SMB200_CTA_PAIR": "0", "SMB200_EXACT_N256": "3"},
-                                 {"SMB200_CTA_PAIR": "1", "SMB200_EXACT_N256": "3"}, {"SMB200_NO_NCAT": "1"}],
-                         ids=["single_cta", "pairs_everywhere", "pairs_128wide", "wide_single", "wide_pairs", "three_mma"])
-def test_conv_tile_variants(env):
-    """The launcher picks the tile (128x128 / 128x256 / CTA-pair 256x256, 256x128) per layer and problem size (the
-    wide / pair tiles only when the 128x128 tiling fills the machine, i.e. not at these test sizes); the switches are
-    read once per process, so every kernel variant is forced in a child process ("wide_pairs" = what the long-K layers
-    run at bench.py's batch; "three_mma" = hi*hi and hi*lo as separate MMAs instead of the concatenated N = 2*BLOCK_N
-    one, in the GEMM and in the resident-patch kernel)."""
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    names = ["1x1_64_256", "1x1_1024_256", "3x3_s2_p0_ds", "3x3_d2_p2", "3x3_p1_ds3", "3x3_p0_kernel", "1x1_mask3969",
-             "3x3_v2", "3x3_p1", "3x3_p1_128_31"]
-    code = _VARIANT_SCRIPT.format(tests=os.path.join(root, "tests"), root=root, names=names)
-    r = subprocess.run([sys.executable, "-c", code], env={**os.environ, **env}, capture_output=True, text=True,
-                       timeout=300)
-    assert r.returncode == 0 and "variants ok" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
-
-
 def test_conv_small_channels_simt_only():
     # Cin not a multiple of 64 has no tensor-core path: the operator must say so, not fall back silently
     x = torch.randn(1, 16, 9, 9).cuda()

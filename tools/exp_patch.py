@@ -1,10 +1,9 @@
-"""Times the bottleneck conv2 shapes through sm_conv2d (exact mode): resident-patch kernel vs im2col kernel
-(SMB200_PATCH3X3=0 in the environment selects the latter).  Used under ncu for the source-level stall picture."""
-import os, sys, torch
+"""Runs the bottleneck conv2 shapes through sm_conv2d (exact mode) on the resident-patch kernel.  Used under ncu for
+the source-level stall picture."""
+import sys, torch
 sys.path.insert(0, '.')
 import siammask_b200 as smb
 dev = 'cuda'
-mode = os.environ.get("SMB200_PATCH3X3", "1")
 for (B, C, H) in [(64, 64, 63), (64, 128, 31)]:
     g = torch.Generator().manual_seed(0)
     x = torch.randn(B, C, H, H, generator=g).to(dev)
@@ -13,4 +12,4 @@ for (B, C, H) in [(64, 64, 63), (64, 128, 31)]:
     for _ in range(3):
         out = smb.conv2d(x, w, sc, sh, 1, 1, 1, relu=True)
     torch.cuda.synchronize()
-    print(f"mode {mode} B={B} C={C} H={H} ok {tuple(out.shape)}", flush=True)
+    print(f"B={B} C={C} H={H} ok {tuple(out.shape)}", flush=True)

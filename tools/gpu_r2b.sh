@@ -1,11 +1,6 @@
 #!/bin/bash
-# r02: descriptor base-offset experiment for the resident-patch 3x3 kernel + bulk xcorr tests, then the r2a sequence
+# r02: bulk xcorr tests, then the r2a sequence
 mkdir -p gpurun_out
-for mode in 1 2; do
-  echo "=== SMB200_PATCH3X3=$mode" >> gpurun_out/r2b_patch.log
-  ( SMB200_PATCH3X3=$mode timeout 600 python -m pytest tests/test_gpu_ops.py -m gpu -q -p no:cacheprovider -k "3x3_p1" 2>&1 | tail -25 ) >> gpurun_out/r2b_patch.log 2>&1
-done
-grep -E "===|passed|failed|parity\]" gpurun_out/r2b_patch.log | tail -40
 ( timeout 600 python -m pytest tests/test_gpu_ops.py -m gpu -q -p no:cacheprovider -k "xcorr" 2>&1 | tail -15 ) > gpurun_out/r2b_xcorr.log 2>&1
 tail -4 gpurun_out/r2b_xcorr.log
 bash tools/gpu_r2a.sh

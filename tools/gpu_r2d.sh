@@ -1,5 +1,5 @@
 #!/bin/bash
-# r02: convergent-issue GEMM kernels — op tests, shape tests, whole GPU suite, tracker tests, bench, A/B launch lists
+# r02: convergent-issue GEMM kernels — op tests, shape tests, whole GPU suite, tracker tests, bench with launch list
 mkdir -p gpurun_out
 ( timeout 900 python -m pytest tests/test_gpu_ops.py -m gpu -q -x -p no:cacheprovider 2>&1 | tail -15 ) > gpurun_out/r2d_ops.log 2>&1
 tail -3 gpurun_out/r2d_ops.log
@@ -9,5 +9,3 @@ tail -5 gpurun_out/r2d_shapes.log
 tail -3 gpurun_out/r2d_pytest.log
 timeout 1200 python bench.py --steps 20 --warmup 3 --dump-layers gpurun_out/r2d_layers.tsv > gpurun_out/r2d_bench.json 2> gpurun_out/r2d_bench.err
 tail -3 gpurun_out/r2d_bench.err; cut -c1-300 gpurun_out/r2d_bench.json
-SMB200_PATCH3X3=0 timeout 900 python bench.py --steps 20 --warmup 3 --no-cpu --no-context --no-verify --dump-layers gpurun_out/r2d_layers_nopatch.tsv > gpurun_out/r2d_bench_nopatch.json 2> gpurun_out/r2d_bench_nopatch.err
-cut -c1-200 gpurun_out/r2d_bench_nopatch.json

@@ -2,9 +2,3 @@
 mkdir -p gpurun_out
 timeout 600 ncu --set full --clock-control none --import-source on --kernel-name-base demangled -k regex:xcorr_nhwc -s 4 -c 1 -f -o gpurun_out/prof_xcorr_nhwc_r02 python bench.py --steps 1 --warmup 3 --min-seconds 0 --no-cpu --no-context --no-verify --no-loop > gpurun_out/r2h_ncu_xcorr.log 2>&1
 tail -2 gpurun_out/r2h_ncu_xcorr.log | cut -c1-200
-for v in 0 1; do
-SMB200_NCHW_WIDE=$v timeout 600 python bench.py --steps 20 --warmup 3 --no-cpu --no-context --no-verify --no-loop --min-seconds 1 --dump-layers gpurun_out/r2h_layers_nchw$v.tsv > gpurun_out/r2h_nchw$v.json 2> gpurun_out/r2h_nchw$v.err
-python -c "
-import json; d=json.load(open('gpurun_out/r2h_nchw$v.json')); print('nchw_wide=$v', round(d['value']), round(d['ms_per_step'],3), d['clocks']['sm_mhz'])"
-grep "mask.head.3" gpurun_out/r2h_layers_nchw$v.tsv | cut -f1,3,6
-done
